@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W           # our CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --gpus N ...           # the reference's CPU implementation (oracle port)
+    python bench.py ... --dump-outputs DIR                  # also save the last timed step's outputs (DIR/bon.npy, cor.npy)
 
 One "step" = one forward over one batch of 32 synthetic panoramas per GPU (BASELINE.json configs[1];
 N>1 = configs[3]: data-parallel shards + one NCCL all-gather of the outputs per step).
@@ -29,6 +30,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True        # the benchmark runs from a built tree and writes nothing into it
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
@@ -418,6 +420,8 @@ def run_ours(args):
         return float(ms.item()), int(launches.item()), prof, sampler.summary(), last
 
     total_ms, launches, _, clocks, last_pipe = timed(True, False)          # 1. headline
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_pipe)
     serial_ms, _, prof, clocks_serial, last_serial = timed(False, True)    # 2. serial + per-launch events
     value = world * BATCH * args.steps / (total_ms * 1e-3)
 
@@ -609,6 +613,16 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(path, outputs):
+    """--dump-outputs: the (bon, cor) the headline path returned in its last timed step -- with N>1 the all-gathered
+    result -- as float32 path/bon.npy [B,2,1024] and path/cor.npy [B,1,1024] (393 KB per 32 panoramas).  Weights and
+    inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in zip(('bon', 'cor'), outputs):
+        np.save(os.path.join(path, name + '.npy'), t.detach().float().cpu().numpy())
+
+
 def train_step_aux(dev, batch=8, steps=3):
     """One optimizer step of train.py (:272-281) through the library's autograd boundary: train-mode forward with tape,
     L1 + BCE-with-logits (train.py:53-56), loss.backward() (hn_train_backward + one gradient per parameter),
@@ -719,7 +733,13 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-comparators', action='store_true', help='skip the PyTorch-eager GPU comparator')
     ap.add_argument('--quick-cpu', action='store_true', help='CPU baseline: bs1 only')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step to DIR/bon.npy and DIR/cor.npy (float32)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs applies to --impl ours')
     if args.impl == 'reference':
         run_reference(args)
     else:

@@ -3,8 +3,9 @@
 Run in the build container only (the GPU box has no /root/reference):
     python tests/golden/make_golden.py
 Outputs (committed): tests/golden/forward_identity.npz, forward_randombn.npz,
-panostretch_small.npz, panostretch_rows.npz, tta_randombn.npz, augment.npz (row f3), rotate.npz (row f4),
-train_all.npz / train_frozen1.npz (row f1, train-mode forward), train_backward.npz / train_backward_frozen1.npz (row f1, loss.backward()).  The two shims are the ones SURVEY.md section 8c
+panostretch_small.npz + panostretch_small_kx_above_1.npz, panostretch_rows.npz, tta_randombn.npz, augment.npz (row f3), rotate.npz (row f4),
+train_all.npz / train_frozen1.npz (row f1, train-mode forward), train_backward.npz / train_backward_frozen1.npz (row f1, loss.backward()),
+checkpoint_ref_utils.json (save_model / load_trained_model on our class).  The two shims are the ones SURVEY.md section 8c
 describes: torchvision.resnet50 is forced to weights=None (no network), nothing else is patched.
 Weights/inputs come from horizonnet_b200.weights (numpy RandomState => reproducible on any box).
 """
@@ -78,7 +79,10 @@ def golden_panostretch():
             small[f'cor_{kx}_{ky}'] = c
     o0, _ = ref_ps.pano_stretch(img_s, cs, 1.5, 0.75, order=0)
     small['out0_1.5_0.75'] = o0
+    # two files of under 1 MB each: the kx > 1 half of the grid goes to the second
+    upper = {k: small.pop(k) for k in list(small) if k.split('_')[0] in ('out', 'cor') and float(k.split('_')[1]) > 1.0}
     np.savez_compressed(os.path.join(HERE, 'panostretch_small.npz'), **small)
+    np.savez_compressed(os.path.join(HERE, 'panostretch_small_kx_above_1.npz'), **upper)
 
     rows = {}
     img = np.random.RandomState(0).random_sample((512, 1024, 3)).astype(np.float32)
@@ -347,7 +351,44 @@ def golden_train_backward(name='backward', freeze_earlier_blocks=-1, batch=2, ws
     print('train backward golden', name, ': loss', loss.item(), 'parameters with a gradient:', len(names), 'oracle autograd vs reference, worst tensor (rel. to its max):', worst)
 
 
+def state_dict_digests(sd):
+    """[key, shape, dtype, sha256 of the raw bytes] of every tensor, in the state_dict's order."""
+    import hashlib
+    return [[k, list(v.shape), str(v.dtype), hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest()]
+            for k, v in sd.items()]
+
+
+def golden_checkpoint():
+    """The REAL misc/utils.save_model / load_trained_model (utils.py:49-65) applied to our HorizonNet class, unmodified:
+    the layout of the checkpoint save_model wrote (top-level keys, args, kwargs, a digest of every state_dict tensor)
+    and what load_trained_model rebuilt from it."""
+    import json
+    import tempfile
+    import types
+    from misc import utils as ref_utils             # reference misc/utils.py
+    from horizonnet_b200.model import HorizonNet
+    net = HorizonNet('resnet50', True)
+    net.load_state_dict(synthetic_state_dict(4, 'random'), strict=True)
+    with tempfile.TemporaryDirectory() as d:
+        path = os.path.join(d, 'ck.pth')
+        ref_utils.save_model(net, path, types.SimpleNamespace(lr=1e-4))          # args is vars()'d
+        ck = torch.load(path, map_location='cpu')
+        net2 = ref_utils.load_trained_model(HorizonNet, path)                      # strict load
+    saved = state_dict_digests(ck['state_dict'])
+    assert state_dict_digests(net2.state_dict()) == saved
+    out = {'weights_seed': 4, 'bn': 'random', 'top_level': list(ck), 'args': ck['args'], 'kwargs': ck['kwargs'],
+           'loaded': {'class': type(net2).__name__, 'backbone': net2.backbone, 'use_rnn': net2.use_rnn},
+           'state_dict': saved}
+    with open(os.path.join(HERE, 'checkpoint_ref_utils.json'), 'w') as f:         # one line per tensor
+        head = json.dumps({k: v for k, v in out.items() if k != 'state_dict'})
+        f.write(head[:-1] + ',\n"state_dict": [\n' + ',\n'.join(json.dumps(e) for e in saved) + '\n]}\n')
+    print('checkpoint golden', out['top_level'], out['kwargs'], len(saved), 'tensors')
+
+
 if __name__ == '__main__':
+    if len(sys.argv) > 1 and sys.argv[1] == 'checkpoint':  # only the save_model / load_trained_model fixture
+        golden_checkpoint()
+        sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == 'backward':    # only the backward fixtures of row f1
         golden_train_backward()
         golden_train_backward('backward_frozen1', 1)
@@ -370,3 +411,4 @@ if __name__ == '__main__':
     golden_train('frozen1', 1, bn_momentum=0.01)
     golden_train_backward()
     golden_train_backward('backward_frozen1', 1)
+    golden_checkpoint()

@@ -49,27 +49,30 @@ def test_checkpoint_layout_round_trip():
         assert torch.equal(v, sd[k]), k
 
 
-def test_checkpoint_round_trip_through_the_real_reference_utils(tmp_path):
-    """With /root/reference present (build container only): the reference's OWN save_model / load_trained_model
-    (misc/utils.py:49-65) applied to our class, unmodified."""
-    ref = '/root/reference'
-    if not os.path.isdir(ref):
-        pytest.skip('reference checkout not present on this box')
-    import importlib.util
-    import types
-    spec = importlib.util.spec_from_file_location('_ref_utils', os.path.join(ref, 'misc', 'utils.py'))
-    utils = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(utils)
-    sd = synthetic_state_dict(4, 'random')
+def test_checkpoint_round_trip_through_the_real_reference_utils(golden_dir, tmp_path):
+    """The reference's OWN save_model / load_trained_model (misc/utils.py:49-65) applied to our class, unmodified, as
+    recorded in tests/golden/checkpoint_ref_utils.json (make_golden.py golden_checkpoint): the same weights give the
+    kwargs and the tensors (key, shape, dtype, sha256 of the bytes) save_model stored, and a checkpoint of the layout it
+    wrote loads back into our class the way load_trained_model does it."""
+    import hashlib
+    import json
+
+    def state_dict_digests(sd):                     # same record as make_golden.py state_dict_digests
+        return [[k, list(v.shape), str(v.dtype), hashlib.sha256(v.detach().contiguous().numpy().tobytes()).hexdigest()]
+                for k, v in sd.items()]
+    g = json.load(open(os.path.join(golden_dir, 'checkpoint_ref_utils.json')))
     net = HorizonNet('resnet50', True)
-    net.load_state_dict(sd, strict=True)
+    net.load_state_dict(synthetic_state_dict(g['weights_seed'], g['bn']), strict=True)
+    assert {'backbone': net.backbone, 'use_rnn': net.use_rnn} == g['kwargs']          # utils.py:49-58 reads these
+    assert state_dict_digests(net.state_dict()) == g['state_dict']
+    assert g['loaded'] == {'class': 'HorizonNet', 'backbone': 'resnet50', 'use_rnn': True}
     path = str(tmp_path / 'ck.pth')
-    utils.save_model(net, path, types.SimpleNamespace(lr=1e-4))          # utils.py:49-58 (args is vars()'d)
-    net2 = utils.load_trained_model(HorizonNet, path)                      # utils.py:61-65 (strict load)
-    assert isinstance(net2, HorizonNet) and net2.backbone == 'resnet50' and net2.use_rnn is True
-    assert list(net2.state_dict().keys()) == list(sd.keys())
-    for k, v in net2.state_dict().items():
-        assert torch.equal(v, sd[k]), k
+    parts = {'args': g['args'], 'kwargs': g['kwargs'], 'state_dict': net.state_dict()}
+    torch.save(OrderedDict((k, parts[k]) for k in g['top_level']), path)
+    ck = torch.load(path, map_location='cpu')
+    net2 = HorizonNet(**ck['kwargs'])                                                  # utils.py:61-65 (strict load)
+    net2.load_state_dict(ck['state_dict'])
+    assert state_dict_digests(net2.state_dict()) == g['state_dict']
 
 
 def test_train_mode_never_runs_the_eval_graph():

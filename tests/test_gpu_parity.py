@@ -377,7 +377,8 @@ def test_tta_forward_matches_reference_golden_and_oracle(golden_dir):
 
 # ------------------------------------------------------------------------------- pano_stretch
 def test_pano_stretch_small_grid_vs_golden(golden_dir):
-    g = np.load(os.path.join(golden_dir, 'panostretch_small.npz'))
+    g = dict(np.load(os.path.join(golden_dir, 'panostretch_small.npz')))
+    g.update(np.load(os.path.join(golden_dir, 'panostretch_small_kx_above_1.npz')))
     img = g['img']
     for kx in KGRID:
         for ky in KGRID:

@@ -57,7 +57,8 @@ def test_forward_oracle_rejects_other_sizes():
 
 
 def test_panostretch_oracle_small_full_grid(golden_dir):
-    g = np.load(os.path.join(golden_dir, 'panostretch_small.npz'))
+    g = dict(np.load(os.path.join(golden_dir, 'panostretch_small.npz')))
+    g.update(np.load(os.path.join(golden_dir, 'panostretch_small_kx_above_1.npz')))
     img = g['img']
     for kx in KGRID:
         for ky in KGRID:
