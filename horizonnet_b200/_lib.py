@@ -60,6 +60,10 @@ SIGNATURES = {
     'hn_model_submit_host': (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int]),
     'hn_model_collect_host': (ctypes.c_int, [vp, vp, vp]),
     'hn_model_infer_tta': (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, c_int_p, ctypes.c_int, vp, vp, vp]),
+    'hn_layout_workspace_bytes': (ctypes.c_longlong, [ctypes.c_int]),
+    'hn_layout': (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, ctypes.c_float, ctypes.c_int] + [vp] * 8),
+    'hn_model_infer_layout': (ctypes.c_int, [vp, vp, ctypes.c_int, ctypes.c_int, c_int_p, ctypes.c_int, ctypes.c_int,
+                                             ctypes.c_float, ctypes.c_int] + [vp] * 10),
     'hn_model_stage': (ctypes.c_int, [vp, ctypes.c_char_p, vp, ctypes.c_longlong, c_int_p, vp]),
     'hn_model_set_option': (ctypes.c_int, [vp, ctypes.c_char_p, ctypes.c_int]),
     'hn_model_check': (ctypes.c_int, [vp]),

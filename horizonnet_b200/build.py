@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'lib', 'libhorizonnet_b200.so')
-SOURCES = ['model.cu', 'conv_f32.cu', 'conv_tc.cu', 'tail.cu', 'lstm.cu', 'lstm_cluster.cu', 'panostretch.cu', 'rotate.cu', 'tta.cu', 'train_fwd.cu', 'bwd_kernels.cu', 'wgrad_tc.cu', 'train_step.cu']
+SOURCES = ['model.cu', 'conv_f32.cu', 'conv_tc.cu', 'tail.cu', 'lstm.cu', 'lstm_cluster.cu', 'panostretch.cu', 'rotate.cu', 'tta.cu', 'layout.cu', 'train_fwd.cu', 'bwd_kernels.cu', 'wgrad_tc.cu', 'train_step.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '-cudart', 'static']
 

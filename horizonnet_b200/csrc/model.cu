@@ -783,9 +783,56 @@ int hn_model_infer_tta(hn_model* m, const float* x, int in_channels, int flip, c
     for (int i = 0; i < n_rotate; ++i, ++v) { host[v] = 2; host[64 + v] = shifts[i]; }   // 'rotate shift' (:39-42)
     HN_CUDA_OK(cudaMemcpyAsync(m->tta_ints, host, sizeof(host), cudaMemcpyHostToDevice, st));
     HN_CUDA_OK(cudaStreamSynchronize(st));                      // host[] is a stack array
-    if (tta_views(x, m->x_slot[1], V, m->tta_ints, m->tta_ints + 64, st)) return -1;
+    if (tta_views(x, m->x_slot[1], 1, V, m->tta_ints, m->tta_ints + 64, st)) return -1;
     if (hn_model_forward(m, m->x_slot[1], V, 3, m->bon_out, m->cor_out, st)) return -1;
-    return tta_merge(m->bon_out, m->cor_out, V, m->tta_ints, m->tta_ints + 64, y_bon_pix, y_cor, st);
+    return tta_merge(m->bon_out, m->cor_out, 1, V, m->tta_ints, m->tta_ints + 64, y_bon_pix, y_cor, st);
+}
+
+long long hn_layout_workspace_bytes(int B) { return B >= 1 ? (long long)hn::layout_workspace_bytes(B) : 0; }
+
+int hn_layout(const float* y_bon_pix, const float* y_cor, int B, int mode, float min_v, int r_px, void* workspace,
+              float* cor_id, int* n_cor, float* z1, int* status, int* peaks, int* types, void* stream) {
+    HN_CHECK(y_bon_pix && y_cor && workspace && cor_id && n_cor && z1 && status, "hn_layout: NULL argument");
+    HN_CHECK(B >= 1 && B <= 65535, "hn_layout: batch must be in 1..65535");
+    HN_CHECK(mode >= HN_LAYOUT_GENERAL && mode <= HN_LAYOUT_RAW, "hn_layout: mode must be general, cuboid or raw");
+    HN_CHECK(mode == HN_LAYOUT_RAW || r_px >= 1, "hn_layout: the peak window r_px must be >= 1");
+    return layout(y_bon_pix, y_cor, B, mode, min_v, r_px, workspace, cor_id, n_cor, z1, status, peaks, types,
+                  (cudaStream_t)stream);
+}
+
+int hn_model_infer_layout(hn_model* m, const float* x, int B, int flip, const int* shifts, int n_rotate, int mode,
+                          float min_v, int r_px, void* workspace, float* y_bon_pix, float* y_cor, float* cor_id,
+                          int* n_cor, float* z1, int* status, int* peaks, int* types, void* stream) {
+    HN_CHECK(m && x && y_bon_pix && y_cor, "hn_model_infer_layout: NULL argument");
+    HN_CHECK(B >= 1, "hn_model_infer_layout: batch must be >= 1");
+    HN_CHECK(n_rotate >= 0 && n_rotate <= 32 && (n_rotate == 0 || shifts), "hn_model_infer_layout: bad rotate list");
+    const int V = 1 + (flip ? 1 : 0) + n_rotate;
+    HN_CHECK(V <= m->max_batch, "hn_model_infer_layout: views exceed max_batch");
+    HN_CHECK(m->submit_count == m->collect_count, "hn_model_infer_layout: collect the submitted batches first");
+    HN_ON_DEVICE(m->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    int host[128];
+    int v = 0;
+    host[v] = 0; host[64 + v] = 0; ++v;                         // same view list as hn_model_infer_tta
+    if (flip) { host[v] = 1; host[64 + v] = 0; ++v; }
+    for (int i = 0; i < n_rotate; ++i, ++v) { host[v] = 2; host[64 + v] = shifts[i]; }
+    HN_CUDA_OK(cudaMemcpyAsync(m->tta_ints, host, sizeof(host), cudaMemcpyHostToDevice, st));
+    HN_CUDA_OK(cudaStreamSynchronize(st));                      // host[] is a stack array
+    const int chunk = m->max_batch / V;                         // chunk * V views per forward
+    const size_t per = (size_t)3 * 512 * 1024;
+    for (int b0 = 0; b0 < B; b0 += chunk) {
+        const int nb = B - b0 < chunk ? B - b0 : chunk;
+        const float* xin = x + b0 * per;
+        if (V > 1) {
+            if (tta_views(xin, m->x_slot[1], nb, V, m->tta_ints, m->tta_ints + 64, st)) return -1;
+            xin = m->x_slot[1];
+        }
+        if (hn_model_forward(m, xin, nb * V, 3, m->bon_out, m->cor_out, st)) return -1;
+        if (tta_merge(m->bon_out, m->cor_out, nb, V, m->tta_ints, m->tta_ints + 64, y_bon_pix + (size_t)b0 * 2 * 1024,
+                      y_cor + (size_t)b0 * 1024, st))
+            return -1;
+    }
+    return hn_layout(y_bon_pix, y_cor, B, mode, min_v, r_px, workspace, cor_id, n_cor, z1, status, peaks, types, stream);
 }
 
 int hn_model_stage(hn_model* m, const char* stage, float* out, long long capacity, int dims[4], void* stream) {

@@ -19,9 +19,12 @@ int linear_head(const float* rnn, const float* w, const float* bias, float* bon,
 int lstm_layer(const float* xproj, const float* w_hh_fwd, const float* w_hh_bwd, float* out, int T, int B,
                void* scratch, int* error_flag, cudaStream_t st);
 size_t lstm_scratch_bytes();
-int tta_views(const float* x, float* views, int V, const int* modes_dev, const int* shifts_dev, cudaStream_t st);
-int tta_merge(const float* bon, const float* cor, int V, const int* modes_dev, const int* shifts_dev, float* y_bon,
+int tta_views(const float* x, float* views, int B, int V, const int* modes_dev, const int* shifts_dev, cudaStream_t st);
+int tta_merge(const float* bon, const float* cor, int B, int V, const int* modes_dev, const int* shifts_dev, float* y_bon,
               float* y_cor, cudaStream_t st);
+size_t layout_workspace_bytes(int B);
+int layout(const float* y_bon_pix, const float* y_cor, int B, int mode, float min_v, int r_px, void* workspace,
+           float* cor_id, int* n_cor, float* z1, int* status, int* peaks, int* types, cudaStream_t st);
 int pano_stretch_device(const float* img, float* out, int n, int H, int W, int C, const double* kx_dev,
                         const double* ky_dev, double* scratch, int order, cudaStream_t st);
 int pano_stretch_device_f64(const double* img, double* out, int n, int H, int W, int C, const double* kx_dev,

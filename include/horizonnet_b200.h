@@ -146,6 +146,45 @@ int hn_model_collect_host(hn_model* m, float* bon_host, float* cor_host);
 int hn_model_infer_tta(hn_model* m, const float* x_dev, int in_channels, int flip, const int* shifts_host,
                        int n_rotate, float* y_bon_pix_dev, float* y_cor_dev, void* stream);
 
+/* Room-layout post-processing on the device (reference inference.py:21-29 find_N_peaks and :95-139 with the
+ * misc/post_proc.py functions they call: floor/ceiling plane, wall-wall peaks, wall fitting, the Polygon validity
+ * check with its cuboid fallback, corner assembly).  One CTA per panorama; every input and output is on the device.
+ *   y_bon_pix [B][2][1024]  boundary rows in pixels and y_cor [B][1024] corner probabilities, exactly what
+ *                           hn_model_infer_tta / hn_model_infer_layout write (inference.py:90-93);
+ *   mode                    HN_LAYOUT_GENERAL, HN_LAYOUT_CUBOID (force_cuboid) or HN_LAYOUT_RAW (force_raw);
+ *   min_v                   peak threshold (the caller applies the reference's default: 0 cuboid, 0.05 general);
+ *   r_px                    peak window int(round(W * r / 2)) (inference.py:108; 26 for the default r = 0.05);
+ *   workspace               hn_layout_workspace_bytes(B) bytes of device memory (no allocation inside);
+ *   cor_id [B][HN_LAYOUT_MAX_COR][2]  normalised (u, v) corners, n_cor[B] rows valid per panorama;
+ *   z1 [B]                  the floor plane (np_refine_by_fix_z, float32);
+ *   status [B][4]           {HN_LAYOUT_OK / HN_LAYOUT_ASSERT / HN_LAYOUT_RING, fell back to the cuboid (1/0),
+ *                            number of peaks, number of walls}; ASSERT = the reference raises AssertionError
+ *                            (gen_ww_cuboid / gen_ww_general / vote asserts), RING = the reference raises ValueError
+ *                            (a wall ring shapely cannot build); cor_id is empty for both;
+ *   peaks [B][1024], types [B][HN_LAYOUT_MAX_WALLS]  (optional, NULL to skip) the peak columns and wall types
+ *                            (0: x = const, 1: y = const) of the final result. */
+#define HN_LAYOUT_GENERAL 0
+#define HN_LAYOUT_CUBOID 1
+#define HN_LAYOUT_RAW 2
+#define HN_LAYOUT_OK 0
+#define HN_LAYOUT_ASSERT 1
+#define HN_LAYOUT_RING 2
+#define HN_LAYOUT_MAX_WALLS 2048
+#define HN_LAYOUT_MAX_COR 4096
+long long hn_layout_workspace_bytes(int batch);
+int hn_layout(const float* y_bon_pix_dev, const float* y_cor_dev, int batch, int mode, float min_v, int r_px,
+              void* workspace_dev, float* cor_id_dev, int* n_cor_dev, float* z1_dev, int* status_dev, int* peaks_dev,
+              int* types_dev, void* stream);
+
+/* Batched test-time augmentation + forward + layout in one call: x [batch][3][512][1024] on the device, views as in
+ * hn_model_infer_tta (view-major order v * batch + b, chunked so that chunk * views <= max_batch), the merged
+ * signals go to y_bon_pix_dev [batch][2][1024] / y_cor_dev [batch][1024], then hn_layout with the remaining
+ * arguments.  With batch 1 the signals are the bits hn_model_infer_tta writes. */
+int hn_model_infer_layout(hn_model* m, const float* x_dev, int batch, int flip, const int* shifts_host, int n_rotate,
+                          int mode, float min_v, int r_px, void* workspace_dev, float* y_bon_pix_dev, float* y_cor_dev,
+                          float* cor_id_dev, int* n_cor_dev, float* z1_dev, int* status_dev, int* peaks_dev,
+                          int* types_dev, void* stream);
+
 /* Test hook: copies an intermediate result of the LAST forward, converted to the reference's
  * layout, into `out_dev` (fp32).  Stages: "stem" (conv1+bn1+relu, NCHW [B,64,256,512], model.py:73-75),
  * "layer1".."layer4" (NCHW [B,C,H,W], model.py:78-81),
